@@ -25,6 +25,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the bench writes nothing into the tree it runs from (which may be read-only)
 
 import torch  # noqa: E402
 
@@ -92,86 +93,15 @@ def log(msg):
 
 
 def cpu_oracle_subprocess(threads, reps, timeout_s=420):
-    """Runs cpu_reference_step in a child process under a timeout so a slow host cannot stall the GPU bench line.
-    Returns (frames/s, seconds per pass, sample description, kind)."""
+    """Runs cpu_oracle_step in a child process under a timeout so a slow host cannot stall the GPU bench line.
+    Returns (frames/s, seconds per pass, sample description)."""
     code = (f"import sys, json; sys.path.insert(0, {ROOT!r}); import bench; "
-            f"print(json.dumps(bench.cpu_reference_step({threads}, 4, {reps})))")
+            f"print(json.dumps(bench.cpu_oracle_step({threads}, 4, {reps})))")
     try:
-        r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=timeout_s)
+        r = subprocess.run([sys.executable, "-B", "-c", code], capture_output=True, text=True, timeout=timeout_s)
         return tuple(json.loads(r.stdout.strip().splitlines()[-1]))
     except Exception as e:  # timeout / parse error
-        return None, None, f"cpu baseline unavailable: {type(e).__name__}", "port"
-
-
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")  # unmodified reference files of the path (oracle/make_ref.py; git-ignored, travels)
-
-
-def reference_available() -> bool:
-    return os.path.exists(os.path.join(REF_DIR, "MANIFEST.json")) and os.path.exists(os.path.join(REF_DIR, "models", "arch", "SpatialNet.py"))
-
-
-def reference_modules(num_layers=None):
-    """The reference's own SpatialNet / STFT / Norm objects (imported from baseline/_ref, unmodified) carrying the oracle's synthetic
-    parameters, plus TrainModule.forward (SharedTrainer.py:104-132) restated around them — 12 lines without arithmetic of their own;
-    SharedTrainer.py itself needs pytorch_lightning, which the image does not have."""
-    from oracle import spatialnet_oracle as O
-    if REF_DIR not in sys.path:
-        sys.path.insert(0, REF_DIR)
-    from models.arch.SpatialNet import SpatialNet as RefNet  # noqa: E402  (reference)
-    from models.io.norm import Norm as RefNorm  # noqa: E402
-    from models.io.stft import STFT as RefSTFT  # noqa: E402
-    cfg = dict(O.SMALL_CFG) if num_layers is None else dict(O.SMALL_CFG, num_layers=num_layers)
-    arch = RefNet(dim_input=cfg["dim_input"], dim_output=cfg["dim_output"], dim_squeeze=cfg["dim_squeeze"], num_layers=cfg["num_layers"],
-                  num_freqs=cfg["num_freqs"], encoder_kernel_size=5, dim_hidden=cfg["dim_hidden"], dim_ffn=cfg["dim_ffn"],
-                  num_heads=cfg["num_heads"], kernel_size=(5, 3), conv_groups=(8, 8))
-    arch.load_state_dict({k: v.clone() for k, v in O.synth_params(cfg, 2).items()}, strict=True)
-    stft, norm = RefSTFT(n_fft=CFG["n_fft"], n_hop=CFG["hop"]), RefNorm(mode="frequency")
-
-    def train_module_forward(x, ref_channel=0):  # SharedTrainer.py:104-132 with channels = all, loss.mask None
-        X, stft_paras = stft.stft(x)
-        B, C, F, T = X.shape
-        X, (Xr, XrMM) = norm.norm(X, ref_channel=ref_channel)
-        X = X.permute(0, 2, 3, 1)
-        X = torch.view_as_real(X).reshape(B, F, T, -1)
-        out = arch(X)
-        if not torch.is_complex(out):
-            out = torch.view_as_complex(out.float().reshape(B, F, T, -1, 2))
-        out = out.permute(0, 3, 1, 2)
-        Yr_hat = norm.inorm(out, (Xr, XrMM))
-        return stft.istft(Yr_hat, stft_paras)
-
-    return arch, train_module_forward
-
-
-def cpu_reference_step(threads, b=4, reps=2):
-    """One training pass of the path on the host cores through the UNMODIFIED reference modules when baseline/_ref holds them
-    (kind "reference"), else through the op-set port (kind "port").  Returns (frames/s, seconds, sample description, kind)."""
-    if not reference_available():
-        return cpu_oracle_step(threads, b, reps) + ("port",)
-    try:
-        from oracle import eager_gpu as E
-        torch.set_num_threads(threads)
-        arch, fwd = reference_modules()
-        x, tgt = synth_batch(b, 1234)
-        ts = []
-        for i in range(reps + 1):
-            t0 = time.perf_counter()
-            arch.zero_grad(set_to_none=True)
-            est = fwd(x)
-            loss = E.neg_si_sdr_pit2(est, tgt)  # torchmetrics (models/io/loss.py) is absent: the oracle's pinned restatement
-            loss.backward()
-            ts.append(time.perf_counter() - t0)
-            if sum(ts) > 120:  # bounded sample: stop once ~2 minutes of CPU work have been spent
-                break
-        timed = ts[1:] if len(ts) > 1 else ts
-        t = min(timed)
-        note = f"1 warm-up + {len(ts) - 1} timed (best)" if len(ts) > 1 else "single cold pass (host too slow for a warm-up within the bound)"
-        return (b * CFG["T"] / t, t, f"B={b} utterance(s) x T=250 frames, wave->wave fwd+bwd through the unmodified reference modules "
-                f"(baseline/_ref: models.arch.SpatialNet, models.io.stft / norm; TrainModule.forward glue and the torchmetrics loss restated), "
-                f"{threads} threads, {note}", "reference")
-    except Exception as e:  # a broken copy must not take the arm down: fall back to the port and say so
-        fps, t, sample = cpu_oracle_step(threads, b, reps)
-        return fps, t, sample + f" [baseline/_ref failed: {type(e).__name__}: {e}]"[:300], "port"
+        return None, None, f"cpu baseline unavailable: {type(e).__name__}"
 
 
 def cpu_oracle_step(threads, b=4, reps=2):
@@ -462,14 +392,14 @@ def run_reference(args):
         return
     cores = min(os.cpu_count() or 1, 32)
     steps = max(1, min(args.steps, 3))
-    fps, t, sample, kind = cpu_reference_step(cores, b=4, reps=steps)
+    fps, t, sample = cpu_oracle_step(cores, b=4, reps=steps)
     _emit(json.dumps({
         "impl": "reference", "metric": "T-F frames/sec (SpatialNet-small 6ch F=129, training step fwd+bwd incl. STFT/iSTFT)",
         "value": fps, "unit": "frames/s", "n_gpus": args.gpus, "steps": steps, "warmup": 1, "ms_per_step": t * 1e3,
         "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": "SpatialNet-small 6ch F=129 T=250 fwd+bwd, batch=32 (BASELINE configs[1])", "global_batch": 32,
                    "cpu_sample_batch": 4, "frames_per_utt": CFG["T"]},
-        "cpu_baseline": {"value": fps, "unit": "frames/s", "cores": cores, "kind": kind, "sample": sample},
+        "cpu_baseline": {"value": fps, "unit": "frames/s", "cores": cores, "kind": "port", "sample": sample},
         "e2e": {"value": fps, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "rtf": t / (4 * TS / 8000.0),
     }))
@@ -498,7 +428,11 @@ def main():
     ap.add_argument("--profile", action="store_true", help="1 warm-up + 1 step only (for ncu); prints no bench line")
     ap.add_argument("--layers", type=int, default=CFG["L"], help="number of SpatialNet layers (profiling only; default 8)")
     ap.add_argument("--no-graphs", action="store_true", help="launch every kernel eagerly instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (estimates, loss, flat gradient, "
+                    "updated parameters; rank 0) to DIR/<name>.npy in float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly ONE line, the JSON result: everything else that a library writes to file descriptor 1 (NCCL's
     # version banner, for one) is routed to stderr, and the JSON line goes to the saved original stdout
     global _JSON_OUT
@@ -560,7 +494,7 @@ def main():
         est = pipe(x)
         loss = neg_si_sdr_pit(est, y)[0]
         loss.backward()
-        return loss
+        return loss, est
 
     def reduce_grads():
         if world > 1:
@@ -574,10 +508,10 @@ def main():
         opt.step()
 
     def step(x, y):  # eager step
-        loss = fwd_bwd(x, y)
+        loss, est = fwd_bwd(x, y)
         reduce_grads()
         opt_step()
-        return loss
+        return loss, est
 
     graphs = {}
 
@@ -589,24 +523,24 @@ def main():
         gA = torch.cuda.CUDAGraph()
         ops.LAUNCHES = 0
         with torch.cuda.graph(gA):
-            lossA = fwd_bwd(x_st, y_st)
+            lossA, estA = fwd_bwd(x_st, y_st)
         graphs["launches"] = ops.LAUNCHES
         gH = torch.cuda.CUDAGraph()
         with torch.cuda.graph(gH, pool=gA.pool()):
             x_st.copy_(x_host, non_blocking=True)
             y_st.copy_(y_host, non_blocking=True)
-            lossH = fwd_bwd(x_st, y_st)
+            lossH, estH = fwd_bwd(x_st, y_st)
             loss_host.copy_(lossH.detach().reshape(1), non_blocking=True)
         gB = torch.cuda.CUDAGraph()
         with torch.cuda.graph(gB, pool=gA.pool()):
             opt_step()
-        graphs.update(A=gA, H=gH, B=gB, lossA=lossA, lossH=lossH)
+        graphs.update(A=gA, H=gH, B=gB, lossA=lossA, lossH=lossH, estA=estA, estH=estH)
 
     def gstep(host_io):
         (graphs["H"] if host_io else graphs["A"]).replay()
         reduce_grads()
         graphs["B"].replay()
-        return graphs["lossH"] if host_io else graphs["lossA"]
+        return (graphs["lossH"], graphs["estH"]) if host_io else (graphs["lossA"], graphs["estA"])
 
     def timed(nsteps, host_io):
         if world > 1:
@@ -616,21 +550,21 @@ def main():
         e0.record()
         for _ in range(nsteps):
             if use_graphs:
-                loss = gstep(host_io)
+                loss, est = gstep(host_io)
             elif host_io:
                 x = x_host.to(dev, non_blocking=True)
                 y = y_host.to(dev, non_blocking=True)
-                loss = step(x, y)
+                loss, est = step(x, y)
                 loss_host.copy_(loss.detach().reshape(1), non_blocking=True)
             else:
-                loss = step(x_dev, y_dev)
+                loss, est = step(x_dev, y_dev)
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.barrier()
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item()) / nsteps, float(loss.detach())
+        return float(ms.item()) / nsteps, loss.detach(), est.detach()
 
     if args.profile:
         step(x_dev, y_dev)
@@ -664,10 +598,16 @@ def main():
     if rank == 0:
         sampler.start()
     ops.LAUNCHES = 0
-    ms_dev, loss_v = timed(args.steps, host_io=False)
+    ms_dev, loss_t, est_t = timed(args.steps, host_io=False)
+    loss_v = float(loss_t)
     log(f"device-resident: {ms_dev:.2f} ms/step")
+    if args.dump_outputs and rank == 0:
+        # the outputs of the last timed step, taken before any later pass moves the parameters on (about 18 MB at batch 32)
+        dump = {"estimates": est_t, "loss": loss_t.reshape(1), "grad_flat": net._last_flat_grad,
+                "params_flat": torch.cat([p.detach().reshape(-1) for p in params])}
+        dump = {k: v.float().cpu().numpy() for k, v in dump.items()}
     launches = graphs["launches"] if use_graphs else ops.LAUNCHES // args.steps
-    ms_e2e, _ = timed(args.steps, host_io=True)
+    ms_e2e, _, _ = timed(args.steps, host_io=True)
     log(f"e2e: {ms_e2e:.2f} ms/step")
     clocks = sampler.stop() if rank == 0 else None
 
@@ -755,8 +695,14 @@ def main():
     if world == 1 and not args.no_cpu_baseline:
         cores = min(os.cpu_count() or 1, 32)
         log(f"cpu baseline on {cores} threads")
-        fps, t, sample, kind = cpu_oracle_subprocess(cores, reps=2)
-        out["cpu_baseline"] = {"value": fps, "unit": "frames/s", "cores": cores, "kind": kind, "sample": sample}
+        fps, t, sample = cpu_oracle_subprocess(cores, reps=2)
+        out["cpu_baseline"] = {"value": fps, "unit": "frames/s", "cores": cores, "kind": "port", "sample": sample}
+    if args.dump_outputs:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, v in dump.items():
+            np.save(os.path.join(args.dump_outputs, k + ".npy"), v)
     _emit(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()

@@ -20,14 +20,21 @@ def _net(cfg, P):
     return net
 
 
+def _x(z):
+    """The seeded input of tests/golden/online_f9_t270.npz (make_golden_online.py), checked against its stored sum."""
+    x = torch.randn(2, 9, 270, 12, generator=torch.Generator().manual_seed(270))
+    assert abs(x.double().sum().item() - float(z["x_sum"])) < 1e-6, "torch's seeded generator no longer gives the stored input"
+    return x
+
+
 @pytest.mark.gpu
 def test_online_matches_reference_golden():
     """The unmodified reference's own output (T = 270 > 251: causal attention over all past frames, the function torch executes)."""
     z = np.load(os.path.join(G, "online_f9_t270.npz"))
-    P = {k[2:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("P.")}
     cfg = dict(O.SMALL_CFG, num_layers=2, num_freqs=9)
+    P = O.synth_params(cfg, 107)
     net = _net(cfg, P)
-    y = net(torch.from_numpy(z["x"]).cuda())
+    y = net(_x(z).cuda())
     torch.cuda.synchronize()
     net.check_device_errors()
     e = O.rel_l2(y.cpu(), torch.from_numpy(z["y"]))
@@ -39,10 +46,10 @@ def test_online_matches_reference_golden():
 def test_online_window_ring_wraps():
     """window=True: the key/value ring of 251 frames wraps at T = 270; against the oracle with the mask the reference builds."""
     z = np.load(os.path.join(G, "online_f9_t270.npz"))
-    P = {k[2:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("P.")}
     cfg = dict(O.SMALL_CFG, num_layers=2, num_freqs=9)
+    P = O.synth_params(cfg, 107)
     net = _net(cfg, P)
-    x = torch.from_numpy(z["x"])
+    x = _x(z)
     y = net(x.cuda(), window=True)
     with torch.no_grad():
         ref = OO.online_forward({k: v.double() for k, v in P.items()}, x.double(), cfg, scope=251)
@@ -104,7 +111,7 @@ def test_online_state_dict_matches_reference_names():
     cfg = dict(O.SMALL_CFG, num_layers=2, num_freqs=9)
     net = OnlineSpatialNet(dim_input=12, dim_output=4, num_layers=2, dim_squeeze=8, num_freqs=9, dim_hidden=96, dim_ffn=192, num_heads=4)
     z = np.load(os.path.join(G, "online_f9_t270.npz"))
-    ref_keys = {k[2:]: z[k].shape for k in z.files if k.startswith("P.")}
+    ref_keys = {k[6:]: tuple(z[k]) for k in z.files if k.startswith("shape.")}
     sd = net.state_dict()
     assert set(sd.keys()) == set(ref_keys.keys())
     for k, shp in ref_keys.items():
